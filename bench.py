@@ -43,7 +43,26 @@ def parse_args():
     ap.add_argument("--backbone", default=None, help="r50_tile workload backbone: r50 (default) | r101 | swin_tiny")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-graph", dest="no_graph", action="store_true", help="r50_tile: eager launches instead of a CUDA graph")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", dest="dump_outputs", default=None, metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy (float32 or "
+                         "float64, at most 64 MiB in all); the inputs are seeded, so two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_LIMIT = 64 << 20                                              # bytes --dump-outputs writes at most
+
+
+def write_outputs(path, arrays):
+    """--dump-outputs: every array as path/<name>.npy, float32 as it is and anything else as float64"""
+    arrays = {k: np.asarray(v) for k, v in arrays.items()}
+    arrays = {k: (a if a.dtype == np.float32 else a.astype(np.float64)) for k, a in arrays.items()}
+    assert sum(a.nbytes for a in arrays.values()) <= DUMP_LIMIT
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 # ----------------------------------------------------------------------------------------------- clocks
@@ -157,7 +176,8 @@ FP32_PEAK_TFLOPS = 148 * 128 * 2 * 1.965e9 / 1e12      # 148 SMs x 128 FMA lanes
 
 
 def time_nms(dets_h, local, steps, warm, world, flush, thr=0.1):
-    """device-timed rotated NMS of one box set resident in HBM: (ms per call, sweep-kernel ms, kept, stats)"""
+    """device-timed rotated NMS of one box set resident in HBM: (ms per call, sweep-kernel ms, kept, stats, kept indices of
+    the last call)"""
     import torch
     from orientedreppoints_b200 import _lib
     from orientedreppoints_b200.ops import rnms_indices
@@ -178,7 +198,8 @@ def time_nms(dets_h, local, steps, warm, world, flush, thr=0.1):
         sweep.append(_lib.last_sweep_ms())
     _lib.set_timing(False)
     ms = max_over_ranks(sum(a.elapsed_time(b) for a, b in ev) / steps, world)
-    return ms, float(np.mean(sweep)), int(cnt.item()), _lib.last_nms_stats()
+    kept = int(cnt.item())
+    return ms, float(np.mean(sweep)), kept, _lib.last_nms_stats(), keep[:kept].cpu().numpy()
 
 
 def nms_sweep(args, rank, world, local, sizes=(10000, 20000, 50000, 100000, 200000)):
@@ -196,7 +217,7 @@ def nms_sweep(args, rank, world, local, sizes=(10000, 20000, 50000, 100000, 2000
     for n in sizes:
         for dense in (False, True):
             d = gen_rotated_boxes(n, seed=100 + rank, extent=1024.0 if dense else const_density_extent(n))
-            ms, sweep_ms, kept, st = time_nms(d, local, 5, 3, world, flush)
+            ms, sweep_ms, kept, st, _ = time_nms(d, local, 5, 3, world, flush)
             pairs = n * (n - 1) / 2.0
             row = {"n": n, "variant": "dense_1024" if dense else "const_density", "ms": ms, "Mpairs_per_s": world * pairs / (ms * 1e-3) / 1e6,
                    "kept": kept, "sweep_kernel_ms": sweep_ms, "pairs_swept": st["pairs_total"], "pairs_aabb": st["pairs_aabb"],
@@ -260,9 +281,11 @@ def run_nms(args, rank, world, local, dense=True):
     if rank == 0:
         sampler.start()
     _lib.reset_launch_count()
-    ms, sweep_avg, kept, stats = time_nms(dets_h, local, args.steps, max(args.warmup, 3), world, flush, thr)
+    ms, sweep_avg, kept, stats, keep = time_nms(dets_h, local, args.steps, max(args.warmup, 3), world, flush, thr)
     launches = _lib.launch_count()
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        write_outputs(args.dump_outputs, {"keep": keep})
     pairs = n * (n - 1) / 2.0
     for _ in range(2):
         poly_gpu_nms(dets_h, thr, device_id=local)

@@ -133,10 +133,6 @@ def nms_f32(dets, thresh, guard=False):
 
 
 # ----------------------------------------------------------------------------- compiled reference
-def ref_available():
-    return os.path.exists(os.path.join(REF_DIR, "libref_polyiou.so"))
-
-
 def ref_polyiou():
     if "poly" not in _REF:
         l = ctypes.CDLL(os.path.join(REF_DIR, "libref_polyiou.so"))

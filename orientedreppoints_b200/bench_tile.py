@@ -85,12 +85,14 @@ def _device_steps(det, img, steps, warm, world, flush, benchmod, use_graph, samp
     """`steps` device-resident steps (dense graph -> fused post-processing -> packed detections -> all-gather), CUDA events
     around every step, L2 flush between steps.  The collective is asynchronous: step s waits for the gather of step s-1
     (the last step also for its own), so the ranks are not forced into lockstep and the gather overlaps the next step's
-    dense graph.  Returns (ms per step as max over ranks, per-tile detection counts, launches counted by the library)."""
+    dense graph.  Returns (ms per step as max over ranks, per-tile detection counts, launches counted by the library,
+    (dets, labels, counts) as simple_test returned them in the last step)."""
     from . import gather as G
     pending = [None]
+    out = [None]
 
     def step(last=False):
-        dets, labels, counts = det.simple_test(img, return_tensors="padded")
+        dets, labels, counts = out[0] = det.simple_test(img, return_tensors="padded")
         buf, _ = G.pack(dets, labels, counts)
         h = G.all_gather_detections(buf, async_op=True)
         res = pending[0].wait() if pending[0] is not None else None
@@ -121,7 +123,22 @@ def _device_steps(det, img, steps, warm, world, flush, benchmod, use_graph, samp
     benchmod.barrier(world)
     launches = _lib.launch_count()
     total_ms = benchmod.max_over_ranks(sum(a.elapsed_time(b) for a, b in ev), world)
-    return total_ms / steps, [int(v) for v in all_cnt.reshape(-1).tolist()], launches
+    return total_ms / steps, [int(v) for v in all_cnt.reshape(-1).tolist()], launches, out[0]
+
+
+def step_outputs(dets, labels, counts, limit):
+    """host copy of what simple_test returned in a step: the valid detections of every tile concatenated in tile order
+    (float32 [sum(counts), 27], the rows the padded output holds), their labels, the per-tile counts and the tile indices.
+    If every tile would take more than `limit` bytes, a fixed, seeded sample of the tiles is kept."""
+    n, cap = dets.shape[0], dets.shape[1]
+    per_tile = cap * (dets.shape[2] * 4 + 8) + 16
+    tiles = np.arange(n)
+    if n * per_tile > limit:
+        tiles = np.sort(np.random.RandomState(0).choice(n, limit // per_tile, replace=False))
+    cnt = counts.cpu().numpy()[tiles]
+    valid = np.arange(cap)[None, :] < cnt[:, None]
+    return {"detections": dets.cpu().numpy()[tiles][valid], "labels": labels.cpu().numpy()[tiles][valid],
+            "counts": cnt, "tiles": tiles}
 
 
 def _roofline_pass(det, img, steps, flush):
@@ -196,7 +213,7 @@ def run_config(backbone, precision, batch, args, rank, world, local, benchmod, f
     g = torch.Generator().manual_seed(1000 + rank)
     img = torch.randint(0, 256, (batch, 1024, 1024, 3), generator=g, dtype=torch.uint8).to(dev)
     steps = steps or max(3, min(args.steps, 10))
-    ms_step, ndet, _ = _device_steps(det, img, steps, 3, world, flush, benchmod, not getattr(args, "no_graph", False))
+    ms_step, ndet, _, _ = _device_steps(det, img, steps, 3, world, flush, benchmod, not getattr(args, "no_graph", False))
     pk = benchmod.peaks()
     fl_tile = swin_flops_per_tile() if depth == "swin_tiny" else conv_flops_per_tile(depth)
     k_ms, k_n, k_fl, _ = _roofline_pass(det, img, steps, flush)
@@ -227,9 +244,11 @@ def run(args, rank, world, local, benchmod):
 
     use_graph = not getattr(args, "no_graph", False)
     sampler = benchmod.ClockSampler(local)
-    ms_step, ndet, launches = _device_steps(det, img, args.steps, warm, world, flush, benchmod, use_graph,
-                                            sampler=sampler if rank == 0 else None)
+    ms_step, ndet, launches, last = _device_steps(det, img, args.steps, warm, world, flush, benchmod, use_graph,
+                                                  sampler=sampler if rank == 0 else None)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        benchmod.write_outputs(args.dump_outputs, step_outputs(*last, benchmod.DUMP_LIMIT))
     # roofline pass
     tc_ms, tc_launches, tc_flops, launches_dense = _roofline_pass(det, img, args.steps, flush)
     if use_graph:

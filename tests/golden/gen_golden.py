@@ -92,6 +92,18 @@ def overlapping_pairs(dets, rng, n_pairs):
     return np.concatenate(p).astype(np.float32), np.concatenate(qq).astype(np.float32)
 
 
+def clustered_pairs():
+    """iou_clustered.npz: 4000 random pairs of object-like clusters (many near-duplicates) through polyiou.cpp (fp64) and
+    rnms_cpu.cpp rotate_iou (fp32)"""
+    d = po.gen_clustered_boxes(40, 12, seed=11)
+    rng = np.random.RandomState(5)
+    i, j = rng.randint(0, len(d), 4000).astype(np.int32), rng.randint(0, len(d), 4000).astype(np.int32)
+    p, q = d[i, :8], d[j, :8]
+    np.savez_compressed(os.path.join(OUT, "iou_clustered.npz"), dets=d, i=i, j=j,
+                        ref64=po.ref_iou_poly_pairs(p, q), ref32=po.ref_rotate_iou_pairs(p, q))
+    print("iou_clustered:", p.shape)
+
+
 def main():
     assert os.path.isdir(REF), "golden vectors can only be minted where /root/reference exists"
     build_ref.build(verbose=True)
@@ -118,6 +130,7 @@ def main():
     assert np.array_equal(swig_check, ref64[:200], equal_nan=True)
     np.savez_compressed(os.path.join(OUT, "iou_pairs.npz"), p=p, q=q, ref64=ref64, ref32=ref32)
     print("iou_pairs:", p.shape, "nonzero", int((ref64 > 1e-9).sum()), "max|f32-f64|", float(np.nanmax(np.abs(ref32 - ref64))))
+    clustered_pairs()
 
     # ---------------------------------------------------------------- NMS, config[0] of BASELINE.json
     def nms_suite(name, d):

@@ -140,6 +140,21 @@ def build_reference_model(ResNet, FPN, Head, depth):
     return m
 
 
+SAMPLE = 4096
+
+
+def store_sampled(out, key, a):
+    """store the output `a` as at most SAMPLE of its elements at fixed, seeded flat positions (key_idx) together with its
+    shape (key_shape): the test still runs the whole graph, and every golden file stays under 1 MB"""
+    if a.size <= SAMPLE:
+        idx = np.arange(a.size)
+    else:
+        idx = np.sort(np.random.RandomState(0).choice(a.size, SAMPLE, replace=False))
+    out[key] = a.reshape(-1)[idx]
+    out[key + "_idx"] = idx.astype(np.int32)
+    out[key + "_shape"] = np.array(a.shape, dtype=np.int64)
+
+
 def main():
     ResNet, FPN, Head = install_stubs()
     out = {}
@@ -157,10 +172,10 @@ def main():
         out[tag + "_meta"] = np.array([depth, seed, h, w], dtype=np.int64)
         out[tag + "_img"] = img.numpy()
         for l in range(5):
-            out["%s_feat%d" % (tag, l)] = feats[l].numpy()
-            out["%s_cls%d" % (tag, l)] = cls[l].numpy()
-            out["%s_init%d" % (tag, l)] = init[l].numpy()
-            out["%s_refine%d" % (tag, l)] = refine[l].numpy()
+            store_sampled(out, "%s_feat%d" % (tag, l), feats[l].numpy())
+            store_sampled(out, "%s_cls%d" % (tag, l), cls[l].numpy())
+            store_sampled(out, "%s_init%d" % (tag, l), init[l].numpy())
+            store_sampled(out, "%s_refine%d" % (tag, l), refine[l].numpy())
         print(tag, [tuple(f.shape) for f in feats], float(feats[0].abs().max()), float(cls[0].abs().max()))
     np.savez_compressed(os.path.join(HERE, "dense_ref.npz"), **out)
     print("wrote dense_ref.npz")

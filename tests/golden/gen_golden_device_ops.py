@@ -14,6 +14,7 @@ import os
 import sys
 
 import numpy as np
+import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
@@ -78,11 +79,17 @@ def main():
         col1, col2 = np.zeros((c * 9, nb, ho, wo)), np.zeros((c * 9, nb, ho, wo))
         rd.ref_deformable_im2col_f64(P(x), P(off), None, nb, c, h, w, 3, 3, p_, s_, d_, P(col1))
         rd.ref_deformable_im2col_f64(P(x), P(off), P(msk), nb, c, h, w, 3, 3, p_, s_, d_, P(col2))
+        # the convolution the columns feed (the GEMM of deform_conv_cuda.cpp:231-236) with 5 output channels
+        wt = torch.randn(5, c, 3, 3, generator=torch.Generator().manual_seed(ci), dtype=torch.float64).numpy()
+        conv = lambda col: (wt.reshape(5, c * 9) @ col.reshape(c * 9, -1)).reshape(5, nb, ho, wo).transpose(1, 0, 2, 3)  # noqa: E731
         dcn.update({"dcn%d_cfg" % ci: np.array([s_, p_, d_]), "dcn%d_x" % ci: x, "dcn%d_off" % ci: off, "dcn%d_mask" % ci: msk,
-                    "dcn%d_col" % ci: col1, "dcn%d_colm" % ci: col2})
-    np.savez_compressed(os.path.join(HERE, "device_ops_ref.npz"), **dcn, mar_pts=pts, mar_boxes=boxes, mar_map=maps, mar_hull_n=hull_n,
-                        cx_pts=p2, cx_quads=q, cx_iou=iou, pn_p=pp, pn_q=qq, pn_iou=pn, po_boxes=b, po_query=qb, po_iou=ov,
-                        po_quads=quads)
+                    "dcn%d_w" % ci: wt, "dcn%d_out" % ci: conv(col1), "dcn%d_outm" % ci: conv(col2)})
+    # stored: the first 4000 point sets, 1000 x 40 convex-IoU pairs and 4000 poly_nms pairs (every constructed special case
+    # is among them), which keeps the file under 1 MB
+    m, k = 4000, 1000
+    np.savez_compressed(os.path.join(HERE, "device_ops_ref.npz"), **dcn, mar_pts=pts[:m], mar_boxes=boxes[:m], mar_map=maps[:m],
+                        mar_hull_n=hull_n[:m], cx_pts=p2[:k], cx_quads=q, cx_iou=iou[:k], pn_p=pp[:m], pn_q=qq[:m], pn_iou=pn[:m],
+                        po_boxes=b, po_query=qb, po_iou=ov, po_quads=quads)
     print("wrote device_ops_ref.npz", boxes.shape, iou.shape)
 
 

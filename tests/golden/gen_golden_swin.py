@@ -67,9 +67,9 @@ def main():
             f = m.neck(c)
         out["c%d_img" % case] = img.numpy()
         for i, t in enumerate(c):
-            out["c%d_stage%d" % (case, i)] = t.numpy()
+            gd.store_sampled(out, "c%d_stage%d" % (case, i), t.numpy())
         for i, t in enumerate(f):
-            out["c%d_fpn%d" % (case, i)] = t.numpy()
+            gd.store_sampled(out, "c%d_fpn%d" % (case, i), t.numpy())
         print(case, [tuple(t.shape) for t in c], [tuple(t.shape) for t in f])
     np.savez_compressed(os.path.join(HERE, "swin_ref.npz"), **out)
     print("wrote swin_ref.npz")
