@@ -366,6 +366,30 @@ int orp_gn_apply_f16x3_multi(int nprob, const orp_gn_problem *probs, int C, int 
 int orp_split_tiles_u8(const uint8_t *img_hwc, int H, int W, int C, const int32_t *origins, int ntiles, int subsize,
                        uint8_t *out, void *stream);
 
+/* Multi-scale tile producer (SplitOnlyImage_multi_process.py:53-58: cv2.resize(img, None, fx=rate, fy=rate,
+ * interpolation=INTER_CUBIC) before the cut).  The arithmetic is OpenCV's portable fixed-point INTER_CUBIC for 8-bit
+ * images (DESIGN.md §2 deviation 7): the scaled size is round_half_even(n * rate); per axis and destination index the
+ * table holds 4 source taps clamped to [0, n_src-1] and 4 int16 weights in units of 1/2048; a pixel is
+ * clamp((sum_k wy_k * sum_j wx_j * src + (1 << 21)) >> 22, 0, 255) in int32.  Rate exactly 1 is the plain crop.
+ * No call synchronises the host or allocates.
+ *
+ * orp_resize_cubic_table: one axis of one rate into caller memory, idx int32 [n_dst, 4] (16-byte aligned) and
+ * w int16 [n_dst, 4] (8-byte aligned); n_dst must equal round_half_even(n_src * rate). */
+#define ORP_RESIZE_MAX_RATES 8
+int orp_resize_cubic_table(int n_src, double rate, int n_dst, int32_t *idx, int16_t *w, void *stream);
+/* ntiles tiles of subsize x subsize pixels, out uint8 [ntiles, subsize, subsize, C] (1 <= C <= 4), each computed straight
+ * from the original image img_hwc [H, W, C]; pixels outside the scaled image are zero.  rates: HOST array [nrates]
+ * (nrates <= ORP_RESIZE_MAX_RATES).  tiles: device int32 [ntiles, 3] = (rate index, left, up) in the scaled image of
+ * that rate, so one batch may mix rates.  xidx/xw (yidx/yw): the width (height) tables of every rate != 1, concatenated
+ * in rate order (rates equal to 1 have no table). */
+int orp_resize_tiles_cubic_u8(const uint8_t *img_hwc, int H, int W, int C, int nrates, const double *rates,
+                              const int32_t *xidx, const int16_t *xw, const int32_t *yidx, const int16_t *yw,
+                              const int32_t *tiles, int ntiles, int subsize, uint8_t *out, void *stream);
+/* the whole image: out uint8 [Hr, Wr, C] with Wr = round_half_even(W * rate), Hr likewise (tables may be NULL when
+ * rate == 1) - cv2.resize(img, None, fx=rate, fy=rate, interpolation=INTER_CUBIC) under the contract above */
+int orp_resize_cubic_u8(const uint8_t *img_hwc, int H, int W, int C, double rate, const int32_t *xidx, const int16_t *xw,
+                        const int32_t *yidx, const int16_t *yw, uint8_t *out, void *stream);
+
 /* ------------------------------------------------------------------------------------------
  * Swin-T backbone pieces (mmdet/models/backbones/swin_transformer.py); the Linear layers are
  * orp_conv2d_bf16 1x1 convolutions (relu = 2 selects the exact GELU epilogue)

@@ -12,6 +12,7 @@ LIB_PATH = os.path.join(_HERE, "lib", "liborp_b200.so")
 ORP_NMS_EXACT64, ORP_NMS_COMPAT32 = 0, 1
 ORP_UNION_NAN_KEEPS, ORP_UNION_GUARD, ORP_UNION_NAN_SUPPRESSES = 0, 1, 2
 ORP_ORDER_INDEX_ASC, ORP_ORDER_SCORE_DESC = 0, 1
+ORP_RESIZE_MAX_RATES = 8
 
 _vp = ctypes.c_void_p
 _i = ctypes.c_int
@@ -95,6 +96,9 @@ SIGNATURES = {
     "orp_stem_s2d_bf16": (_i, [_vp, _i, _i, _i, _vp, _vp]),
     "orp_convex_iou": (_i, [_vp, _i, _vp, _i, _vp, _vp]),
     "orp_split_tiles_u8": (_i, [_vp, _i, _i, _i, _vp, _i, _i, _vp, _vp]),
+    "orp_resize_cubic_table": (_i, [_i, _d, _i, _vp, _vp, _vp]),
+    "orp_resize_tiles_cubic_u8": (_i, [_vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _vp, _vp]),
+    "orp_resize_cubic_u8": (_i, [_vp, _i, _i, _i, _d, _vp, _vp, _vp, _vp, _vp, _vp]),
     "orp_stem_s2d_u8_bf16": (_i, [_vp, _i, _i, _i, _vp, _vp, _i, _vp, _vp]),
     "orp_stem_conv_s2d_bf16": (_i, [_vp, _i, _i, _i, _vp, _vp, _i, _vp, _vp]),
     "orp_maxpool3x3s2_bf16": (_i, [_vp, _i, _i, _i, _i, _vp, _vp]),

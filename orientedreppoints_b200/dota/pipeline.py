@@ -10,7 +10,7 @@ The reference goes through PNG tiles, a pickle and per-class text files between 
 leave HBM and the per-class result lines are merged in memory (the same `merge_lines` the file-based mirror uses).
 """
 from .result_merge import merge_lines
-from .split_tiles import split_image
+from .split_tiles import iter_tiles_multiscale, split_image
 
 # mmdet/datasets/dota.py:8-12
 DOTA_CLASSES = ('plane', 'baseball-diamond', 'bridge', 'ground-track-field', 'small-vehicle', 'large-vehicle', 'ship',
@@ -36,5 +36,19 @@ def detect_image(det, img_u8, name="P0000", rate=1, subsize=1024, gap=200, batch
     results = []
     for i in range(0, tiles.shape[0], batch):
         results.extend(det.simple_test(tiles[i:i + batch]))
+    per_class = task1_lines(results, names)
+    return {cname: merge_lines(lines, merge_thresh) for cname, lines in zip(DOTA_CLASSES, per_class)}
+
+
+def detect_image_multiscale(det, img_u8, name="P0000", rates=(0.5, 1.0, 1.5), subsize=1024, gap=200, batch=16,
+                            merge_thresh=None):
+    """The reference's multi-scale test of one image: tiles of every rate (SplitOnlyImage_multi_process.py splitdata(rate)
+    per rate, here one streaming device producer over the original image) -> detector -> ONE ResultMerge over the tiles
+    of all rates (mergebypoly over the parsed pickle; poly2origpoly divides by each tile's rate).  Returns
+    {class name: [`imgname score x1 y1 x2 y2 x3 y3 x4 y4`, ...]} like detect_image."""
+    results, names = [], []
+    for tiles, tnames, _ in iter_tiles_multiscale(img_u8, name, rates, subsize, gap, batch, device=det.device):
+        results.extend(det.simple_test(tiles))
+        names.extend(tnames)
     per_class = task1_lines(results, names)
     return {cname: merge_lines(lines, merge_thresh) for cname, lines in zip(DOTA_CLASSES, per_class)}
